@@ -15,9 +15,13 @@ scaling (each rank owns its own batch of 8; the path has no data-path collective
             timed region
   roofline  dominant kernel (cost volume): algorithmic bytes / its CUDA-event duration vs measured HBM peak
   cpu_baseline / --impl reference
-            the reference's CPU path — the unmodified est_costvolume_CW from the vendored baseline/_ref (git-ignored copy of
-            /root/reference made by scripts/vendor_ref.sh; travels with the snapshot), else its bit-identical ATen port —
-            timed on this box's host cores on a bounded sample (1-frame batches)
+            the reference's CPU path — its operator sequence as the ATen port oracle/torch_ref.py, pinned bit for bit
+            to the reference's own outputs (tests/test_oracle_golden.py) — timed on this box's host cores on a bounded
+            sample (1-frame batches)
+
+--dump-outputs DIR writes what the last timed step computed, as float32 .npy files: pred_gmm.npy (B,2,H,W), the
+Gaussians after the N_iter iterations, and cost_volume.npy (B,D,H,W), the cost volume of the last iteration.  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -159,16 +163,10 @@ def pin_to_gpu_cpus(index):
 
 
 def reference_ops():
-    """The reference's cost-volume function for the baseline legs: the UNMODIFIED models.submodules.homography
-    .est_costvolume_CW (from /root/reference, or its vendored copy baseline/_ref made by scripts/vendor_ref.sh) when
-    available — kind "reference" — else its bit-identical ATen port oracle/torch_ref.py — kind "port".  The sampler
-    (MAGNET.py:154-156) and the update (MAGNET.py:60-69) are inlined in the reference's forward; they are issued here as
-    the same ATen expressions (oracle/torch_ref.py)."""
+    """The reference's cost-volume function for the baseline legs: its ATen port oracle/torch_ref.py, bit-identical to
+    models.submodules.homography.est_costvolume_CW — kind "port".  The sampler (MAGNET.py:154-156) and the update
+    (MAGNET.py:60-69) are inlined in the reference's forward; they are issued here as the same ATen expressions."""
     from oracle import torch_ref
-    from oracle.ref_loader import load_reference
-    ref = load_reference()
-    if ref is not None:
-        return ref.homography.est_costvolume_CW, "reference", ref.root
     return torch_ref.cost_volume_cw, "port", "oracle/torch_ref.py"
 
 
@@ -217,12 +215,25 @@ def cpu_reference_frames(frames_cfg, steps, warmup, threads=None, budget_s=None)
             if budget_s is not None and time.perf_counter() - t0 > budget_s:
                 break
         dt = time.perf_counter() - t0
-    what = ("unmodified models.submodules.homography.est_costvolume_CW (%s)" % where if kind == "reference"
-            else "ATen port of the reference operator sequence (%s)" % where)
+    what = "ATen port of the reference operator sequence (%s)" % where
     info = {"cores": cores, "os_cpu_count": os.cpu_count(), "frames": done, "seconds": dt, "kind": kind,
             "sample": f"{done} x 1-frame batch of {WORKLOADS[frames_cfg]} (B=1), {N_ITER} iterations each, "
                       f"{what}, {cores} threads"}
     return done / dt, info
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_outputs(out_dir, outputs):
+    """One float32 DIR/<name>.npy per output (every rank computes the same work: rank 0 writes)."""
+    import numpy as np
+    total = sum(t.numel() * 4 for t in outputs.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy().astype(np.float32, copy=False))
 
 
 def run_reference_arm(args, rank):
@@ -251,6 +262,7 @@ def main():
     ap.add_argument("--variant", default="auto", choices=["auto", "direct", "cells", "cells_noreuse", "tma", "mma"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gnet", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy")
     args = ap.parse_args()
 
     from magnet_b200 import dist as md
@@ -380,6 +392,8 @@ def main():
         torch.cuda.synchronize()
         graph_ok = bool(torch.equal(graph_pred, eager_pred))
         ms_total = timed(graph.replay, K, sampler)
+        # the graph's output buffers hold the last timed step's results until the next replay or eager step
+        outputs = {"pred_gmm": graph_pred.cpu(), "cost_volume": cv.cpu()} if args.dump_outputs else None
         own_ms_step = own["ms"] / K
         launches = launches_per_step * K
         # spread: the same K-step region repeated (median / min / max of the max-over-ranks time per step)
@@ -524,6 +538,8 @@ def main():
     if rank != 0:
         md.shutdown()
         return
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     peak, peak_src = measured_peak()
     abytes = algorithmic_bytes(B, V, D, C, HW, fused=True)
     achieved = abytes / (kern_ms * 1e-3) / 1e9

@@ -1,7 +1,8 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (imported from /root/reference).
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (baegwangbin/MaGNet) on the CPU.
 
-Run in the build container only (the GPU box has no /root/reference):
-    python tests/golden/make_golden.py
+    python tests/golden/make_golden.py <MaGNet checkout> [name ...]
+
+With names, only those files are written (e.g. ``reference_module``); the others stay as committed.
 
 Inputs are not stored: they are rebuilt from the seed by magnet_b200.synthetic (numpy Generator
 streams are version-stable); each file carries a sha256 of the inputs so a drifting generator is
@@ -10,7 +11,8 @@ detected instead of silently comparing against the wrong reference output.
 Reference entry points exercised:
   models/submodules/homography.py  est_costvolume_CW (:79), est_costvolume_F (:10)
   models/MAGNET.py                 GNET.forward update equations (:58-70), upsample_depth_via_mask (:15-27),
-                                   MAGNET.depth_sampling (:120-128), the sampler expression (:154-156)
+                                   MAGNET.depth_sampling (:120-128), the sampler expression (:154-156),
+                                   MAGNET.forward (:130-175) with stand-in backbones (reference_module.npz)
 """
 import hashlib
 import os
@@ -19,10 +21,10 @@ import types
 
 import numpy as np
 import torch
+import torch.nn as nn
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = "/root/reference"
 sys.path.insert(0, ROOT)
 
 CASES = {
@@ -52,19 +54,111 @@ def f_planes(n=F_PLANES, d_min=0.5, d_max=8.0):
     return ((bounds[:-1] + bounds[1:]) / 2).astype(np.float32)
 
 
-def main():
-    if not os.path.isdir(REF):
-        raise SystemExit("/root/reference not present: golden vectors can only be generated in the build container")
-    sys.path.insert(0, REF)
+# ---- tests/test_gpu_reference_module.py: the reference's MAGNET.forward on stand-in backbones ---------------------
+# Quarter-resolution grid of the forward case; images are 4x larger.  Weights and images are drawn from fixed seeds
+# (not torch's global RNG), so the reference model here and magnet_b200.MAGNET in the test get identical values.
+FORWARD_CASE = dict(B=2, V=3, D=8, H=24, W=32, C=16, seed=97, depth="smooth", invalid=[(1, 2)])
+FORWARD_ITERS = 2
+FORWARD_SAMPLE = 2048          # full-resolution pixels per prediction kept in the golden file (fixed, seeded)
+F_CASE = dict(B=2, V=2, D=8, H=20, W=28, C=16, seed=98, depth="smooth")
+F_CASE_PLANES = (0.8, 6.0, 12)  # torch.linspace arguments of d_center
+# tests/test_oracle_golden.py: the ATen port against the reference bit for bit (both single-threaded)
+PORT_PIN_CASES = ((11, "random"), (12, "smooth"))
+PORT_PIN_PLANES = (0.5, 7.0, 9)
+
+
+def port_pin_inputs(seed, depth):
+    from magnet_b200.synthetic import make_inputs
+    return make_inputs(B=2, V=2, D=6, H=20, W=28, C=8, seed=seed, depth=depth, invalid=[(0, 1)])
+
+
+class TinyD(nn.Module):
+    """D-Net stand-in: (N,3,H,W) -> (fixed (N,2,H/4,W/4) Gaussians [mu, sigma > 0], (N,256,H/4,W/4) features)."""
+
+    def __init__(self, field):
+        super().__init__()
+        self.b = nn.Conv2d(3, 256, 4, stride=4)
+        self.field = field
+
+    def forward(self, x):
+        return self.field.to(x.device), self.b(x)
+
+
+class TinyF(nn.Module):
+    """F-Net stand-in: (N,3,H,W) -> (N,C,H/4,W/4)."""
+
+    def __init__(self, C):
+        super().__init__()
+        self.c = nn.Conv2d(3, C, 4, stride=4)
+
+    def forward(self, x):
+        return self.c(x)
+
+
+def seed_convs(module, seed):
+    """Every Conv2d of ``module`` (in module order) drawn from U(-1/sqrt(fan_in), 1/sqrt(fan_in)) of a seeded generator."""
+    g = torch.Generator().manual_seed(seed)
+    with torch.no_grad():
+        for m in module.modules():
+            if isinstance(m, nn.Conv2d):
+                bound = 1.0 / float(np.sqrt(m.weight[0].numel()))
+                m.weight.copy_((torch.rand(m.weight.shape, generator=g) * 2 - 1) * bound)
+                m.bias.copy_((torch.rand(m.bias.shape, generator=g) * 2 - 1) * bound)
+
+
+def forward_case():
+    """-> (inputs, ref_img, nghbr_imgs, d_net, f_net) of the forward case, on the CPU."""
+    from magnet_b200.synthetic import make_inputs
+    inp = make_inputs(**FORWARD_CASE)
+    B, V, C = FORWARD_CASE["B"], FORWARD_CASE["V"], FORWARD_CASE["C"]
+    H, W = 4 * FORWARD_CASE["H"], 4 * FORWARD_CASE["W"]
+    g = torch.Generator().manual_seed(FORWARD_CASE["seed"])
+    ref_img = torch.rand(B, 3, H, W, generator=g)
+    nghbr_imgs = torch.rand(V * B, 3, H, W, generator=g)
+    d_net, f_net = TinyD(torch.cat([inp.ref_gmms, inp.nghbr_gmms], 0)), TinyF(C)
+    seed_convs(d_net, 1)
+    seed_convs(f_net, 2)
+    return inp, ref_img, nghbr_imgs, d_net, f_net
+
+
+def seed_head(g_net, mask_head):
+    seed_convs(g_net, 3)
+    seed_convs(mask_head, 4)
+
+
+def forward_sample():
+    """Flat (b, y, x) indices of the full-resolution prediction pixels kept in reference_module.npz."""
+    B, H, W = FORWARD_CASE["B"], 4 * FORWARD_CASE["H"], 4 * FORWARD_CASE["W"]
+    return np.sort(np.random.default_rng(FORWARD_CASE["seed"]).choice(B * H * W, FORWARD_SAMPLE, replace=False))
+
+
+def sample_pixels(pred, idx):
+    """(B,2,H,W) -> (len(idx), 2) values at flat (b, y, x) indices."""
+    B, _, H, W = pred.shape
+    return pred.permute(0, 2, 3, 1).reshape(B * H * W, 2)[torch.as_tensor(idx, device=pred.device)]
+
+
+def import_reference(ref_root):
+    if not os.path.isfile(os.path.join(ref_root, "models", "submodules", "homography.py")):
+        raise SystemExit(f"{ref_root} is not a MaGNet checkout (no models/submodules/homography.py)")
+    sys.path.insert(0, ref_root)
     # utils/utils.py:5-7 imports matplotlib, which is absent; the hot path never touches it.
     for name in ("matplotlib", "matplotlib.pyplot"):
         m = types.ModuleType(name)
         m.use = lambda *a, **k: None
         sys.modules.setdefault(name, m)
+
+
+def main(ref_root, only=()):
+    import_reference(ref_root)
     import models.submodules.homography as refh
     from models.MAGNET import GNET, MAGNET, upsample_depth_via_mask
     from magnet_b200.synthetic import make_inputs
 
+    if only:
+        for name in only:
+            {"reference_module": reference_module, "torch_port_pin": torch_port_pin}[name]()
+        return
     torch.set_num_threads(4)
     for name, kw in CASES.items():
         inp = make_inputs(**kw)
@@ -108,6 +202,83 @@ def main():
                         depth=depth.numpy(), mask=mask.numpy(), up=up.numpy(), **ks)
     print("update / upsample / k_list written")
     camera_prep_and_loss(g)
+    reference_module()
+    torch_port_pin()
+
+
+def reference_module():
+    """The reference's MAGNET.forward (MAGNET.py:130-175) in test mode on stand-in backbones, with its iteration-0 cost
+    volume, and est_costvolume_F (homography.py:10) through the F-Net call of MAGNET_F.forward (MAGNET.py:197-200)."""
+    import models.MAGNET as refm
+    import models.submodules.homography as refh
+    from magnet_b200.synthetic import make_inputs
+    inp, ref_img, nghbr_imgs, d_net, f_net = forward_case()
+    M = refm.MAGNET
+    m = M.__new__(M)                                 # MAGNET.__init__ without its checkpoint loading (MAGNET.py:73-118)
+    nn.Module.__init__(m)
+    m.d_net, m.f_net = d_net.eval(), f_net.eval()
+    m.sampling_range, m.n_samples, m.weighting = 3, FORWARD_CASE["D"], "CW5"
+    m.train_iter = m.test_iter = FORWARD_ITERS
+    m.downsample_ratio = 4
+    m.k_list = M.depth_sampling(m)
+    m.g_net = refm.GNET(ch_in=256 + FORWARD_CASE["D"], ch_out=2)
+    h_dim = 128
+    m.mask_head = nn.Sequential(nn.Conv2d(256, h_dim, 3, padding=1), nn.ReLU(inplace=True),
+                                nn.Conv2d(h_dim, h_dim, 1), nn.ReLU(inplace=True),
+                                nn.Conv2d(h_dim, h_dim, 1), nn.ReLU(inplace=True),
+                                nn.Conv2d(h_dim, 9 * 4 * 4, 1))
+    m.upsample_depth = refm.upsample_depth_via_mask
+    seed_head(m.g_net, m.mask_head)
+    m.eval()
+    seen = []
+    cw = refh.est_costvolume_CW
+
+    def spy(*a, **k):
+        out = cw(*a, **k)
+        seen.append(out.clone())
+        return out
+
+    refh.est_costvolume_CW = spy
+    try:
+        with torch.no_grad():
+            preds = m(ref_img, nghbr_imgs, inp.nghbr_poses, inp.is_valid, inp.cam_intrins, mode="test")
+    finally:
+        refh.est_costvolume_CW = cw
+    idx = forward_sample()
+    fin = make_inputs(**F_CASE)
+    d_center = torch.linspace(*F_CASE_PLANES).view(1, -1, 1, 1)
+    with torch.no_grad():
+        cost_f = refh.est_costvolume_F(d_center, fin.ref_feat, fin.nghbr_feat, fin.R, fin.t, fin.is_valid,
+                                       fin.cam_intrins)
+    np.savez_compressed(os.path.join(HERE, "reference_module.npz"),
+                        digest=np.array(input_digest(inp)), f_digest=np.array(input_digest(fin)),
+                        cost_cw0=seen[0].numpy(), pred=np.stack([sample_pixels(p, idx).numpy() for p in preds]),
+                        pred_absmax=np.array([float(p.abs().max()) for p in preds], dtype=np.float32),
+                        cost_f=cost_f.numpy())
+    print("reference module written:", len(preds), "predictions", tuple(preds[0].shape))
+
+
+def torch_port_pin():
+    """est_costvolume_CW / _F single-threaded: with one thread the ATen kernels give the same bits on AVX2 and
+    AVX-512 hosts, so the ATen port can be pinned to these outputs exactly."""
+    import models.submodules.homography as refh
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)
+    save = {}
+    try:
+        for seed, depth in PORT_PIN_CASES:
+            inp = port_pin_inputs(seed, depth)
+            dc = torch.linspace(*PORT_PIN_PLANES).view(1, -1, 1, 1)
+            save[f"cw_{seed}"] = refh.est_costvolume_CW(inp.depth_volume(), inp.ref_feat, inp.nghbr_feat, inp.ref_gmms,
+                                                        inp.nghbr_gmms, inp.R, inp.t, inp.is_valid, inp.cam_intrins,
+                                                        5).numpy()
+            save[f"f_{seed}"] = refh.est_costvolume_F(dc, inp.ref_feat, inp.nghbr_feat, inp.R, inp.t, inp.is_valid,
+                                                      inp.cam_intrins).numpy()
+            save[f"digest_{seed}"] = np.array(input_digest(inp))
+    finally:
+        torch.set_num_threads(threads)
+    np.savez_compressed(os.path.join(HERE, "torch_port_pin.npz"), **save)
+    print("torch port pin written:", sorted(save))
 
 
 def _camera_prep_case():
@@ -220,4 +391,6 @@ def camera_prep_and_loss(g):
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) < 2:
+        raise SystemExit(__doc__)
+    main(sys.argv[1], sys.argv[2:])

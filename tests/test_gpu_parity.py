@@ -324,20 +324,18 @@ def test_full_size_properties_cfg2(cuda):
 def test_full_size_vs_reference_operator_sequence(cuda, cfg):
     """What bench.py measures, at BASELINE.json's full sizes (configs[1] and configs[2]): the production kernel in BOTH
     depth modes — sampler fused (MAGNET_DEPTH_GAUSS) and drop-in (d_volume) — against the reference's operator
-    sequence (grid_sample / repeat / mul / sum; the unmodified reference function when its sources are available, else
-    its bit-identical ATen port) on the same device, with consistency-mask flip accounting: an element beyond
+    sequence (grid_sample / repeat / mul / sum: the ATen port, bit-identical to the reference on the CPU,
+    test_oracle_golden.py) on the same device, with consistency-mask flip accounting: an element beyond
     1e-4 * max must sit on the hard threshold (margin from the same operators) and their number is budgeted."""
     from oracle import torch_ref
-    from oracle.ref_loader import load_reference
     from tests.util import FLIP_BUDGET, MARGIN_TOL, REL_TOL
     inp = make_config(cfg, seed=1)
     g = inp.to(cuda)
     cam_d = {k: v.to(cuda) for k, v in inp.cam_intrins.items()}
-    ref = load_reference()
-    ref_fn = ref.homography.est_costvolume_CW if ref is not None else torch_ref.cost_volume_cw
     with torch.no_grad():
         dvol = ops.sample_depths(g.ref_gmms, inp.k.tolist())
-        want = ref_fn(dvol, g.ref_feat, g.nghbr_feat, g.ref_gmms, g.nghbr_gmms, g.R, g.t, inp.is_valid, cam_d, inp.thres)
+        want = torch_ref.cost_volume_cw(dvol, g.ref_feat, g.nghbr_feat, g.ref_gmms, g.nghbr_gmms, g.R, g.t, inp.is_valid,
+                                        cam_d, inp.thres)
         margin = torch_ref.cw_threshold_margin(dvol, g.nghbr_gmms, g.R, g.t, inp.is_valid, cam_d, inp.thres)
         plan = magnet_b200.MatchingPlan(g.ref_feat, g.nghbr_feat, g.nghbr_gmms, g.nghbr_poses, inp.is_valid,
                                         inp.cam_intrins, thres=inp.thres)
@@ -351,7 +349,7 @@ def test_full_size_vs_reference_operator_sequence(cuda, cfg):
         bad = diff > REL_TOL * scale
         n_bad = int(bad.sum())
         far = bad & (margin > MARGIN_TOL)
-        print(cfg, name, "reference =", "unmodified" if ref is not None else "ATen port", "max rel on agreeing elements",
+        print(cfg, name, "max rel on agreeing elements",
               float(torch.where(bad, torch.zeros_like(diff), diff).max()) / scale, "flips", n_bad, "of", got.numel())
         assert not bool(far.any()), f"{cfg}/{name}: {int(far.sum())} elements differ and are NOT on the threshold"
         assert n_bad <= FLIP_BUDGET * got.numel(), f"{cfg}/{name}: flip budget exceeded ({n_bad})"
